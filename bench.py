@@ -15,6 +15,8 @@ north_star / C5 at N=1 (fixed per-GPU sizes), C4 as "512 graphs, 2/4 GPU shard" 
 gather" at N=8, both also WITH the gather of the rendered PCM inside the step (all-gather of group k overlapped with the render of
 group k+1).
 --impl reference times the reference's CPU algorithm (the oracle port, all host threads) on the same config and batch size.
+Every timed leg runs --steps steps.  --dump-outputs DIR writes a seeded sample of the C2 PCM the last timed step rendered
+(DIR/c2_pcm.npy): the inputs are the same on every run, so two builds can be compared output for output.
 """
 import argparse
 import ctypes
@@ -36,6 +38,7 @@ METRIC = "offline render-quanta/sec (48kHz stereo, 128-frame)"
 FP64_PEAK_TFLOPS = 148 * 64 * 2 * 1.965e9 / 1e12  # B200 non-tensor FP64 (nominal)
 FP32_PEAK_TFLOPS = 148 * 128 * 2 * 1.965e9 / 1e12  # B200 non-tensor FP32: 148 SMs x 128 lanes x FMA at the 1965 MHz boost clock
 PARKING_GARAGE_IR_FRAMES = 178899  # samples/parking-garage-response.wav (164 363 frames @ 44.1 kHz) resampled to 48 kHz (SURVEY §8a a9)
+DUMP_BYTES = 64 * 10**6  # --dump-outputs: at most this much PCM on disk
 
 
 def load_peaks():
@@ -238,7 +241,7 @@ def measure_workload(pkg, eng, D, oracle, name, build, n_gpu, n_cpu, length, ste
     host = np.zeros((n_gpu, 2, length), np.float32)
     eng.set_option(pkg.OPT_PIPELINE_GROUPS, 0)
     e2e = []
-    for i in range(3):
+    for i in range(1 + steps):
         fresh = [build(eng.backend, g) for g in range(n_gpu)]
         D.barrier()
         t0 = time.perf_counter()
@@ -248,7 +251,7 @@ def measure_workload(pkg, eng, D, oracle, name, build, n_gpu, n_cpu, length, ste
     e2e_s = float(np.median(e2e[1:]))
     out["e2e_value"] = quanta / e2e_s
     out["e2e_ms_per_step"] = e2e_s * 1e3
-    out["e2e_how"] = "one wae_render_batch(HOST) call on fresh graphs, pageable out, median of 2 after 1 warm-up"
+    out["e2e_how"] = f"one wae_render_batch(HOST) call on fresh graphs, pageable out, median of {steps} after 1 warm-up"
     if model is not None:
         out["time_batched_model"] = model
     if oracle is not None and n_cpu > 0 and D.rank == 0:
@@ -377,6 +380,16 @@ def build_c2_batch(pkg, backend, n_graphs, length, seed_base=0, pcm=None):
     return [G.c2_buffer_biquad_gain(pkg, backend, seed_base + g, length, pcm=None if pcm is None else pcm[g]) for g in range(n_graphs)]
 
 
+def dump_pcm(out_dir, pcm):
+    """--dump-outputs: the PCM of the last timed step, [graphs][2][length] float32 as the caller receives it.  At C2 size that is
+    3.84 GB, so whole graphs are sampled, the same seeded choice on every run, up to DUMP_BYTES."""
+    per_graph = pcm[0].nbytes
+    k = min(len(pcm), max(1, (DUMP_BYTES - 4096) // per_graph))  # 4096: room for the .npy header
+    pick = np.sort(np.random.default_rng(0).choice(len(pcm), k, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "c2_pcm.npy"), pcm[pick])
+
+
 def run_reference(args, D):
     """--impl reference: the reference's CPU path (oracle port: the Rust crate cannot be built here, no cargo), same config and the
     same number of graphs per step as the GPU arm, all host threads, one context per worker thread."""
@@ -399,6 +412,8 @@ def run_reference(args, D):
         if step >= args.warmup:
             times.append(secs.value)
         del ctxs
+    if args.dump_outputs:
+        dump_pcm(args.dump_outputs, out)
     t = float(np.mean(times))
     value = n * quanta_per_graph / t
     line = {
@@ -429,6 +444,8 @@ def main():
     ap.add_argument("--bind-numa", type=int, default=1, help="bind every rank's host threads to its GPU's NUMA node (pinned memory local to the GPU)")
     ap.add_argument("--kernel-only", action="store_true", help="tuning runs: only the kernel-only leg of C2 (no e2e legs, no other workloads)")
     ap.add_argument("--extra", type=int, default=1, help="also measure the other BASELINE configs (C3 / C4 / north_star / C5 at N=1; C4 at N=2,4; C5 at N=8)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the PCM the last timed step rendered (rank 0; the "
+                                                          "kernel-only leg of C2) to DIR/c2_pcm.npy, so that two builds can be compared output for output")
     args = ap.parse_args()
 
     D = Dist()
@@ -502,6 +519,8 @@ def main():
     value = total_quanta / (ms_per_step * 1e-3)
     batch.set_timing(False)
     batch.sync()
+    if args.dump_outputs and rank == 0:
+        dump_pcm(args.dump_outputs, batch.fetch())
     if args.kernel_only:
         agg = {}
         for name, ms, _n in stage_times:
@@ -533,10 +552,9 @@ def main():
             del fresh
         return walls
 
-    e2e_steps = max(1, min(args.steps, 5))
-    e2e_walls = oneshot(pageable_out, e2e_steps, max(1, min(args.warmup, 2)))
+    e2e_walls = oneshot(pageable_out, args.steps, max(1, min(args.warmup, 2)))
     e2e_s = float(np.mean(e2e_walls))
-    e2e_pinned_walls = oneshot(pinned_view, max(1, min(args.steps, 3)), 1)
+    e2e_pinned_walls = oneshot(pinned_view, args.steps, 1)
     e2e_pinned_s = float(np.mean(e2e_pinned_walls))
     h2d = stats.asset_bytes * world  # whole job, like `value`: every rank copies its own shard over its own PCIe link
     d2h = out_floats * 4 * world
@@ -548,9 +566,8 @@ def main():
     prepare_ms = (time.perf_counter() - t_prep) * 1e3
     pinned_ptr = ctypes.c_void_p(pinned_out.data_ptr())
     batch_e2e.run_pipelined(pinned_ptr)
-    warm_steps = max(1, min(args.steps, 3))
-    _, warm_wall = timed(lambda: batch_e2e.run_pipelined(pinned_ptr), warm_steps)
-    warm_s = D.max(warm_wall / warm_steps)
+    _, warm_wall = timed(lambda: batch_e2e.run_pipelined(pinned_ptr), args.steps)
+    warm_s = D.max(warm_wall / args.steps)
     batch_e2e.destroy()
 
     # ---- roofline of the dominant kernel (CUDA events around every stage launch, on the launching stream)
@@ -639,7 +656,7 @@ def main():
         if rank == 0 and world == 1 and not args.no_cpu_baseline:
             os.sched_setaffinity(0, all_cpus)
             oracle2 = pkg.context.Backend(pkg.Api(ctypes.CDLL(ge.ORACLE_SO), "wao_"))
-        extra = run_extra_workloads(pkg, eng, D, oracle2, len(all_cpus), max(2, min(args.steps, 5)), load_peaks()[0])
+        extra = run_extra_workloads(pkg, eng, D, oracle2, len(all_cpus), args.steps, load_peaks()[0])
         if line is not None:
             line["other_workloads"] = extra
     if line is not None:
